@@ -61,6 +61,8 @@ def parse_args():
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[1] latency leg, the configs[4] leg and the oracle comparison")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of their final launch (frames and buffer results) to DIR/*.npy")
     return ap.parse_args()
 
 
@@ -497,6 +499,39 @@ def parity_leg(local, args, host, dev_ptr, stride):
             "first_problems": [f"receiver {s}: {p}" for s, p in bad[:3]]}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(d, out_dir: str, prefix: str = "") -> None:
+    """What a caller of the timed path holds after its last launch: every receiver's frames (b200_demod_fetch) and buffer
+    results (b200_demod_buffer_results), one float64 .npy per field (all values are integers below 2^53, or doubles, so
+    the conversion is exact).  Frames of all receivers are concatenated in receiver order and `frame_receiver` says whose
+    each one is.  Receivers are taken in order while the files stay within DUMP_LIMIT_BYTES; `receivers` lists them."""
+    from readsb_b200.abi import BUFRES_DTYPE, FRAME_DTYPE
+    frame_fields = [f for f in FRAME_DTYPE.names if not f.endswith("_")]
+    bufres_fields = [f for f in BUFRES_DTYPE.names if not f.endswith("_")]
+    per_frame = 8 * (1 + sum(int(np.prod(FRAME_DTYPE[f].shape)) for f in frame_fields))
+    per_receiver = 8 * (1 + d.max_buffers_per_run * sum(int(np.prod(BUFRES_DTYPE[f].shape)) for f in bufres_fields))
+    frames, bufres, total = [], [], 0
+    for s in range(d.n_streams):
+        f = d.frames(s)
+        if total + per_receiver + per_frame * len(f) > DUMP_LIMIT_BYTES:
+            break
+        total += per_receiver + per_frame * len(f)
+        frames.append(f)
+        bufres.append(d.buffer_results(s))
+    allf = np.concatenate(frames) if frames else np.zeros(0, FRAME_DTYPE)
+    arrays = {"receivers": np.arange(len(frames)),
+              "frame_receiver": np.repeat(np.arange(len(frames)), [len(f) for f in frames])}
+    arrays.update({f"frame_{f}": allf[f] for f in frame_fields})
+    b = np.stack(bufres) if bufres else np.zeros((0, d.max_buffers_per_run), BUFRES_DTYPE)     # [receiver, buffer]
+    arrays.update({f"bufres_{f}": b[f] for f in bufres_fields})
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{prefix}{name}.npy", np.asarray(a, dtype=np.float64))
+
+
 def b200_arm(args, rank, world, local):
     cpu_pool = None
     if not args.no_cpu and world == 1 and rank == 0:
@@ -604,6 +639,8 @@ def b200_arm(args, rank, world, local):
     k_first = 26 + args.warmup * LPS
     ms, scan_ms, launches, frames, clocks = timed(device_step_async, args.steps * LPS, k_first, pipelined=True, sample=True)
     value = world * step_samples * args.steps / (ms * 1e-3) / 1e6
+    if args.dump_outputs:
+        dump_outputs(d, args.dump_outputs, f"rank{rank}_" if world > 1 else "")
 
     # --- e2e: host buffers through the C ABI ----------------------------------------------------------------------
     e2e = None

@@ -71,7 +71,18 @@ static uint32_t g_crc_tab[256];
 static uint32_t g_bit_syn[112]; /* syndrome of a single set bit i of a 112-bit frame (crc.c:59-64) */
 static int g_crc_ready;
 
+static void build_crc_tab(void) {
+    if (g_crc_tab[1]) return;   /* entry 1 is POLY once built */
+    for (int i = 0; i < 256; i++) {
+        uint32_t c = (uint32_t)i << 16;
+        for (int j = 0; j < 8; j++) c = (c & 0x800000) ? ((c << 1) ^ POLY) : (c << 1);
+        g_crc_tab[i] = c & 0xffffff;
+    }
+}
+
+/* callable first thing in a process: builds the table it reads */
 uint32_t oracle_crc24(const uint8_t *msg, int bits) {
+    build_crc_tab();
     int n = bits / 8;
     uint32_t rem = 0;
     for (int i = 0; i < n - 3; i++)
@@ -81,11 +92,7 @@ uint32_t oracle_crc24(const uint8_t *msg, int bits) {
 
 static void build_crc(void) {
     if (g_crc_ready) return;
-    for (int i = 0; i < 256; i++) {
-        uint32_t c = (uint32_t)i << 16;
-        for (int j = 0; j < 8; j++) c = (c & 0x800000) ? ((c << 1) ^ POLY) : (c << 1);
-        g_crc_tab[i] = c & 0xffffff;
-    }
+    build_crc_tab();
     uint8_t m[14];
     for (int i = 0; i < 112; i++) {
         memset(m, 0, sizeof m);

@@ -95,10 +95,11 @@ def build_oracle() -> None:
 
 
 def build_readsb_pair() -> None:
-    """Where the reference tree is present: the whole reference program, stock (oracle/_ref/readsb_cpu) and linked with
-    integration/readsb_shim.c against libb200demod.so (oracle/_ref/readsb_b200), for tests/test_gpu_shim.py.  Needs
-    build_demod() first.  Test infrastructure, like the rest of oracle/."""
-    if not Path("/root/reference/readsb.c").exists() or not LIB_DEMOD.exists():
+    """Where the reference tree is present (oracle/Makefile decides, REF=<dir>): the whole reference program, stock
+    (oracle/_ref/readsb_cpu) and linked with integration/readsb_shim.c against libb200demod.so (oracle/_ref/readsb_b200),
+    for tests/test_gpu_shim.py; without it the target builds nothing.  Needs build_demod() first.  Test infrastructure,
+    like the rest of oracle/."""
+    if not LIB_DEMOD.exists():
         return
     res = subprocess.run(["make", "-C", str(ROOT / "oracle"), "CC=gcc", "readsb-pair"], capture_output=True, text=True)
     if res.returncode != 0:

@@ -1,9 +1,16 @@
 """Shared comparison helpers for the parity tests (CUDA path vs oracle / reference)."""
 from __future__ import annotations
 
+import functools
+import hashlib
+import json
+from pathlib import Path
+
 import numpy as np
 
 from readsb_b200.abi import FRAME_PARITY_FIELDS, frame_hex
+
+REFERENCE_RUNS = Path(__file__).resolve().parent / "golden" / "reference_runs.json"
 
 BUFRES_FIELDS = ("sample_timestamp", "sum_level", "sum_power", "sum_signal_power", "length", "n_frames",
                  "buffer_seq", "icao_flipped", "demod_preambles", "demod_rejected_bad", "demod_rejected_unknown_icao",
@@ -53,6 +60,28 @@ def diff_stats(a: dict, b: dict, fields=STATS_INT_FIELDS) -> list[str]:
     if a["peak_signal_power"] != b["peak_signal_power"]:
         msgs.append(f"stats peak_signal_power: {a['peak_signal_power']!r} vs {b['peak_signal_power']!r}")
     return msgs
+
+
+def digest(a) -> str:
+    """dtype, shape and SHA-256 of an array's bytes: how tests/golden/reference_runs.json stores a reference output too large
+    to keep whole; equal digests mean bit-identical arrays."""
+    a = np.ascontiguousarray(a)
+    return f"{a.dtype.str}{list(a.shape)}:{hashlib.sha256(a.tobytes()).hexdigest()[:32]}"
+
+
+def record_digests(rec: np.ndarray, fields) -> dict:
+    """One digest per field of a frame / buffer-result array (addr masked as in diff_frames)."""
+    return {f: digest(rec[f] & np.uint32(0xFFFFFF) if f == "addr" else rec[f]) for f in fields}
+
+
+def diff_digests(got: dict, want: dict, what: str = "") -> list[str]:
+    return [f"{what}{k}: {got[k]} vs reference {v}" for k, v in want.items() if got[k] != v]
+
+
+@functools.cache
+def reference_runs() -> dict:
+    """The reference's outputs on the inputs of the reference comparisons (tests/golden/make_reference_runs.py)."""
+    return json.loads(REFERENCE_RUNS.read_text())
 
 
 def crc_ok(frames: np.ndarray) -> np.ndarray:

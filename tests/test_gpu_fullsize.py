@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 from oraclelib import Oracle
-from paritylib import diff_bufres, diff_frames, diff_stats
+from paritylib import diff_bufres, diff_digests, diff_frames, diff_stats, record_digests, reference_runs
 from readsb_b200 import synth
 from readsb_b200.abi import FRAME_DTYPE
 
@@ -149,21 +149,26 @@ def test_dense_tile_takes_slow_path_and_stays_exact(cuda):
         d.close()
 
 
+CONFIG1_REFERENCE_FIELDS = ("timestamp", "crc", "score", "msgtype", "msgbits", "correctedbits", "fix_bit", "msg")
+
+
+def config1_capture():
+    return synth.generate(24_000_000, seed=2024, frames_per_sec=180.0, df_mask=synth.DF17 | synth.DF11 | synth.AP, n_icao=64,
+                          p_bit_error=0.1)
+
+
 def test_config1_ten_second_replay(cuda):
     """BASELINE configs[0]: a 10 s, 2.4 MSPS uc8 capture replayed `--device-type ifile` style (183 full buffers of 131072
-    samples + 1 partial at the default --sdr-buffer-size): CUDA path vs the oracle (and the reference library where present)."""
-    from oraclelib import Reference, have_ref
+    samples + 1 partial at the default --sdr-buffer-size): CUDA path vs the oracle and vs the reference library's frames
+    (stored in tests/golden/reference_runs.json)."""
     from readsb_b200.demod import Demodulator
-    iq = synth.generate(24_000_000, seed=2024, frames_per_sec=180.0, df_mask=synth.DF17 | synth.DF11 | synth.AP, n_icao=64,
-                        p_bit_error=0.1)
+    iq = config1_capture()
     o = Oracle(); fo, bo = o.run_stream(iq, 131072)
     assert len(bo) == 184 and len(fo) > 800
     d = Demodulator(n_streams=1, buf_samples=131072, max_buffers_per_run=8)
     fg, bg = d.replay(iq)
     problems = diff_frames(fg, fo) + diff_bufres(bg, bo) + diff_stats(d.stats(0), o.stats())
     assert not problems, "\n".join(problems)
-    if have_ref():
-        ref = Reference()
-        fr = ref.run_stream(iq, 131072, cap=len(fo) + 100)[0]
-        assert not diff_frames(fg, fr, fields=("timestamp", "crc", "score", "msgtype", "msgbits", "correctedbits", "fix_bit", "msg"))
+    problems = diff_digests(record_digests(fg, CONFIG1_REFERENCE_FIELDS), reference_runs()["config1_ten_second_replay"])
+    assert not problems, "\n".join(problems)
     d.close()

@@ -1,5 +1,5 @@
 """-m "not gpu": the CPU oracle against (a) the committed golden fixtures produced by the reference itself,
-(b) the reference built here as a library when /root/reference is present, (c) known-answer vectors."""
+(b) the stored outputs of the reference built as a library (tests/golden/reference_runs.json), (c) known-answer vectors."""
 import json
 import zlib
 from pathlib import Path
@@ -7,8 +7,8 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from oraclelib import Oracle, Reference, have_ref
-from paritylib import diff_bufres, diff_frames, diff_stats
+from oraclelib import Oracle
+from paritylib import diff_bufres, diff_digests, diff_frames, diff_stats, digest, record_digests, reference_runs
 from readsb_b200 import synth
 
 GOLDEN = sorted(p for p in (Path(__file__).parent / "golden").glob("*.npz") if p.stem not in ("beast_stream", "sc16_converters"))
@@ -146,136 +146,149 @@ def test_empty_and_tiny_buffers():
     assert len(bufres) == 3
 
 
-needs_ref = pytest.mark.skipif(not have_ref(), reason="reference tree not available to build oracle/_ref")
+# What the reference's own demodulator, converters, CRC tables and ICAO filter returned for the inputs of the tests below
+# (tests/golden/make_reference_runs.py runs them where the reference is built as a library, oracle/_ref); the tests hold the
+# oracle to those outputs on machines without the reference tree.
+FRAME_FIELDS = ("timestamp", "j", "crc", "addr", "score", "buffer_seq", "signal_len", "phase", "msgtype", "msgbits", "correctedbits",
+                "fix_bit", "msg")
+LIVE_GEN = {"cfg2": synth.config2_stream, "cfg5": synth.config5_stream, "mixed": synth.mixed_stream}
+LIVE_INPUTS = [("cfg2", 1), ("cfg5", 2), ("mixed", 3), ("mixed", 4)]
+LIVE_BUFS = [65536, 131072]
+# what each demodulate2400() call added to Modes.stats_current (the per-buffer counters of b200_buffer_result)
+LIVE_BUFRES_FIELDS = ("sample_timestamp", "length", "n_frames", "buffer_seq", "icao_flipped", "demod_preambles", "demod_rejected_bad",
+                      "demod_rejected_unknown_icao", "demod_accepted", "demod_preamblePhase", "demod_bestPhase")
+OPTION_CASES = [(58, 0, 1), (58, 1, 0), (40, 1, 1), (120, 1, 1)]
+OPTION_FIELDS = ("timestamp", "crc", "score", "msgtype", "correctedbits", "fix_bit", "msg")
+MODEAC_CASES = [(1, 65536), (2, 131072), (3, 20000)]
+ICAO_TTL_MS = 500           # ms of stream time instead of 60 s, same mechanism
+BUSY_CASES = [(120, 3000.0), (400, 6000.0)]
+BUSY_TTL_MS = 400
+BUSY_FIELDS = ("timestamp", "crc", "addr", "score", "msgtype", "correctedbits", "msg")
+MODEAC_SC16_CASES = [(False, 65536), (True, 20000)]
 
 
-@needs_ref
-def test_reference_tables_match():
-    ref = Reference()
-    assert np.array_equal(ref.lut(), Oracle.lut())
+def table_probes(crc24, diagnose1) -> dict:
+    """crc24 of 200 random messages and diagnose1 of every single-bit syndrome, per frame length."""
     rng = np.random.default_rng(1)
+    out = {}
     for nbits in (56, 112):
-        for _ in range(200):
-            msg = rng.integers(0, 256, nbits // 8, dtype=np.uint8).tobytes()
-            assert ref.crc24(msg) == Oracle.crc24(msg)
+        crcs = [crc24(rng.integers(0, 256, nbits // 8, dtype=np.uint8).tobytes()) for _ in range(200)]
+        diag = []
         for bit in range(nbits):
             m = bytearray(nbits // 8); m[bit >> 3] = 1 << (7 - (bit & 7))
-            syn = Oracle.crc24(bytes(m))
-            assert ref.diagnose1(syn, nbits) == Oracle.diagnose1(syn, nbits)
+            diag.append(diagnose1(Oracle.crc24(bytes(m)), nbits))
+        out[str(nbits)] = {"crc24": crcs, "diagnose1": diag}
+    return out
 
 
-@needs_ref
-@pytest.mark.parametrize("kind,seed", [("cfg2", 1), ("cfg5", 2), ("mixed", 3), ("mixed", 4)])
-@pytest.mark.parametrize("buf", [65536, 131072])
+def test_reference_tables_match():
+    assert digest(Oracle.lut()) == reference_runs()["tables"]["lut"]
+    assert table_probes(Oracle.crc24, Oracle.diagnose1) == reference_runs()["tables"]["probes"]
+
+
+@pytest.mark.parametrize("kind,seed", LIVE_INPUTS)
+@pytest.mark.parametrize("buf", LIVE_BUFS)
 def test_oracle_matches_reference_live(kind, seed, buf):
-    gen = {"cfg2": synth.config2_stream, "cfg5": synth.config5_stream, "mixed": synth.mixed_stream}[kind]
-    iq = gen(seed, 1_500_000)
-    ref, o = Reference(), Oracle()
-    fr, levels, br, ml, mp = ref.run_stream(iq, buf)
-    fo, bo = o.run_stream(iq, buf)
-    problems = diff_frames(fo, fr, fields=("timestamp", "j", "crc", "addr", "score", "buffer_seq", "signal_len", "phase",
-                                           "msgtype", "msgbits", "correctedbits", "fix_bit", "msg"))
-    assert not problems, "\n".join(problems)
-    assert np.array_equal(fo["sigpow_sum"] / 65535.0 / 65535.0 / fo["signal_len"], levels)
-    sr, dr = ref.stats()
+    want = reference_runs()[f"live/{kind}/{seed}/{buf}"]
+    o = Oracle()
+    fo, bo = o.run_stream(LIVE_GEN[kind](seed, 1_500_000), buf)
+    problems = diff_digests(record_digests(fo, FRAME_FIELDS), want["frames"], "frames ")
+    problems += diff_digests({"signal_level": digest(fo["sigpow_sum"] / 65535.0 / 65535.0 / fo["signal_len"]),
+                              "mean_level": digest(bo["sum_level"] / 65536.0 / bo["length"])}, want["levels"])
+    problems += diff_digests(record_digests(bo, LIVE_BUFRES_FIELDS), want["bufres"], "bufres ")
     so = o.stats()
-    sr["sum_signal_power"] = so["sum_signal_power"]       # the reference keeps this one as fp64 only
-    assert not diff_stats(so, sr)
-    assert np.array_equal(bo["sum_level"] / 65536.0 / bo["length"], ml)
-    # what each demodulate2400() call added to Modes.stats_current (the per-buffer counters of b200_buffer_result)
-    assert not diff_bufres(bo, br, fields=("sample_timestamp", "length", "n_frames", "buffer_seq", "icao_flipped", "demod_preambles", "demod_rejected_bad",
-                                           "demod_rejected_unknown_icao", "demod_accepted", "demod_preamblePhase", "demod_bestPhase"))
+    problems += diff_stats(so, dict(want["stats"], sum_signal_power=so["sum_signal_power"]))   # the reference keeps this one as fp64 only
+    assert not problems, "\n".join(problems)
 
 
-@needs_ref
-@pytest.mark.parametrize("thr,nfix,fixdf", [(58, 0, 1), (58, 1, 0), (40, 1, 1), (120, 1, 1)])
+def options_input():
+    return synth.mixed_stream(9, 1_000_000)
+
+
+@pytest.mark.parametrize("thr,nfix,fixdf", OPTION_CASES)
 def test_oracle_matches_reference_options(thr, nfix, fixdf):
-    iq = synth.mixed_stream(9, 1_000_000)
-    ref, o = Reference(thr, nfix, fixdf), Oracle(thr, nfix, fixdf)
-    fr = ref.run_stream(iq, 65536)[0]
-    fo = o.run_stream(iq, 65536)[0]
-    problems = diff_frames(fo, fr, fields=("timestamp", "crc", "score", "msgtype", "correctedbits", "fix_bit", "msg"))
-    assert len(fr) > 50 and not problems, "\n".join(problems)
+    want = reference_runs()[f"options/{thr}/{nfix}/{fixdf}"]
+    fo = Oracle(thr, nfix, fixdf).run_stream(options_input(), 65536)[0]
+    problems = diff_digests(record_digests(fo, OPTION_FIELDS), want["frames"])
+    assert want["n_frames"] > 50 and not problems, "\n".join(problems)
 
 
-@needs_ref
-@pytest.mark.parametrize("seed,buf", [(1, 65536), (2, 131072), (3, 20000)])
+@pytest.mark.parametrize("seed,buf", MODEAC_CASES)
 def test_oracle_modeac_matches_reference_live(seed, buf):
-    iq = synth.modeac_stream(seed, 1_500_000)
-    ref, o = Reference(), Oracle()
-    ar, ao = ref.run_stream_ac(iq, buf), o.run_stream_ac(iq, buf)
-    assert len(ar) > 80 and len(ar) == len(ao)
-    assert np.array_equal(ar["timestamp"], ao["timestamp"]) and np.array_equal(ar["modeac"], ao["modeac"])
-    assert ref.modeac_count() == o.stats()["demod_modeac"] == len(ar)
+    want = reference_runs()[f"modeac/{seed}/{buf}"]
+    o = Oracle()
+    ao = o.run_stream_ac(synth.modeac_stream(seed, 1_500_000), buf)
+    assert want["n"] > 80 and len(ao) == want["n"] == want["modeac_count"] == o.stats()["demod_modeac"]
+    problems = diff_digests(record_digests(ao, ("timestamp", "modeac")), want["replies"])
+    assert not problems, "\n".join(problems)
 
 
-@needs_ref
+def icao_ttl_input():
+    return synth.generate(6_000_000, seed=77, frames_per_sec=40, df_mask=synth.DF17 | synth.AP, n_icao=2)
+
+
 def test_icao_ttl_two_flips():
     """An address added by a clean DF17 lives until the second filter flip (SURVEY.md 8a, ICAO-filter timing)."""
-    ttl = 500   # ms of stream time instead of 60 s, same mechanism
-    iq = synth.generate(6_000_000, seed=77, frames_per_sec=40, df_mask=synth.DF17 | synth.AP, n_icao=2)
-    ref, o = Reference(icao_ttl_ms=ttl), Oracle(icao_ttl_ms=ttl)
-    fr = ref.run_stream(iq, 131072)[0]
-    fo, bo = o.run_stream(iq, 131072)
-    assert not diff_frames(fo, fr, fields=("timestamp", "msg", "score"))
+    fo, bo = Oracle(icao_ttl_ms=ICAO_TTL_MS).run_stream(icao_ttl_input(), 131072)
+    assert not diff_digests(record_digests(fo, ("timestamp", "msg", "score")), reference_runs()["icao_ttl_two_flips"])
     assert bo["icao_flipped"].sum() >= 3
 
 
-@needs_ref
+def icao_filter_probes(f) -> list[str]:
+    """Random add / test / expire sequences on one ICAO filter; per step, a digest of the answers to 700 tests."""
+    rng = np.random.default_rng(11)
+    pool = rng.choice(1 << 24, size=6000, replace=False).astype(np.uint32)
+    known, out = [], []
+    for step in range(40):
+        for a in rng.choice(pool, size=int(rng.integers(1, 700))):
+            f.icao_add(int(a)); known.append(int(a))
+        probe = list(rng.choice(pool, size=300)) + known[-200:] + known[:200]
+        out.append(digest(np.array([f.icao_test(int(a)) for a in probe])))
+        if rng.random() < 0.35:
+            f.icao_expire()
+    return out
+
+
+def older_generation_is_forgotten(f):
+    """An address of the older generation dies with the 86th new address of the next one."""
+    f.icao_add(0xABCDEF); f.icao_expire()
+    for a in range(1, 86):
+        f.icao_add(a)
+    assert f.icao_test(0xABCDEF)
+    f.icao_add(86)
+    assert not f.icao_test(0xABCDEF) and f.icao_test(1) and f.icao_test(86)
+
+
 def test_icao_filter_resize_forgets_the_older_generation():
     """icao_filter.c:112-130: once the active generation holds more than buckets / 3 addresses (86, 171, 342 ... from 2^8
     buckets) icaoFilterResize re-inserts the ACTIVE generation only (:66-92) - whatever the older one held is gone; and
     icaoFilterExpire halves the tables when the active generation is small (:97-99).  The oracle's sets follow the same
     state machine: random add / test / expire sequences against the reference's own icao_filter.c."""
-    rng = np.random.default_rng(11)
-    ref, o = Reference(), Oracle()
-    pool = rng.choice(1 << 24, size=6000, replace=False).astype(np.uint32)
-    known = []
-    for step in range(40):
-        for a in rng.choice(pool, size=int(rng.integers(1, 700))):
-            ref.icao_add(int(a)); o.icao_add(int(a)); known.append(int(a))
-        probe = list(rng.choice(pool, size=300)) + known[-200:] + known[:200]
-        got_r = [ref.icao_test(int(a)) for a in probe]
-        got_o = [o.icao_test(int(a)) for a in probe]
-        assert got_r == got_o, f"step {step}"
-        if rng.random() < 0.35:
-            ref.icao_expire(); o.icao_expire()
-    # the advisor's case, spelled out: an address of the older generation dies with the 86th new address of the next one
-    ref, o = Reference(), Oracle()
-    for f in (ref, o):
-        f.icao_add(0xABCDEF); f.icao_expire()
-        for a in range(1, 86):
-            f.icao_add(a)
-        assert f.icao_test(0xABCDEF)
-        f.icao_add(86)
-        assert not f.icao_test(0xABCDEF) and f.icao_test(1) and f.icao_test(86)
+    got, want = icao_filter_probes(Oracle()), reference_runs()["icao_filter_probes"]
+    assert got == want, f"first differing step: {next(i for i, (a, b) in enumerate(zip(got, want)) if a != b)}"
+    older_generation_is_forgotten(Oracle())          # the reference passes the same check (make_reference_runs.py)
 
 
-@needs_ref
-@pytest.mark.parametrize("n_icao,fps", [(120, 3000.0), (400, 6000.0)])
+def busy_input(n_icao, fps):
+    return synth.generate(5_000_000, seed=5, frames_per_sec=fps, df_mask=synth.DF17 | synth.DF11 | synth.AP | synth.DF11_IID, n_icao=n_icao)
+
+
+@pytest.mark.parametrize("n_icao,fps", BUSY_CASES)
 def test_oracle_matches_reference_in_busy_airspace(n_icao, fps):
     """More aircraft than the reference's filter keeps without resizing (> 85, > 170, > 341): address/parity replies of
     aircraft that only the older generation knew are rejected after a resize (score -1), and the scan goes on where the
     reference's does."""
-    ttl = 400
-    iq = synth.generate(5_000_000, seed=5, frames_per_sec=fps, df_mask=synth.DF17 | synth.DF11 | synth.AP | synth.DF11_IID, n_icao=n_icao)
-    ref, o = Reference(icao_ttl_ms=ttl), Oracle(icao_ttl_ms=ttl)
-    fr = ref.run_stream(iq, 65536)[0]
-    fo, bo = o.run_stream(iq, 65536)
-    problems = diff_frames(fo, fr, fields=("timestamp", "crc", "addr", "score", "msgtype", "correctedbits", "msg"))
-    assert len(fr) > 1000 and not problems, "\n".join(problems)
-    sr = ref.stats()[0]
+    want = reference_runs()[f"busy/{n_icao}/{fps}"]
+    o = Oracle(icao_ttl_ms=BUSY_TTL_MS)
+    fo, bo = o.run_stream(busy_input(n_icao, fps), 65536)
     so = o.stats()
-    sr["sum_signal_power"] = so["sum_signal_power"]
-    assert not diff_stats(so, sr)
+    problems = diff_digests(record_digests(fo, BUSY_FIELDS), want["frames"])
+    problems += diff_stats(so, dict(want["stats"], sum_signal_power=so["sum_signal_power"]))
+    assert want["n_frames"] > 1000 and not problems, "\n".join(problems)
     assert bo["icao_flipped"].sum() >= 3
 
 
-@needs_ref
-@pytest.mark.parametrize("q11", [False, True])
-def test_oracle_sc16_converters_match_reference(q11):
-    """SURVEY 8(f) row 3: convert_sc16_nodc (convert.c:212-250) / convert_sc16q11_nodc (:329-367), magnitudes and the two
-    sequential float accumulators, against the reference's own converters reached through init_converter."""
+def sc16_input(q11):
     rng = np.random.default_rng(5 + q11)
     n = 70001
     lim = 2048 if q11 else 32768
@@ -283,11 +296,18 @@ def test_oracle_sc16_converters_match_reference(q11):
     iq[:64] = [-lim, lim - 1] * 32                       # saturating corner: magsq clamps at 1
     iq[64:128] = 0
     iq[128:4000] = rng.integers(-lim // 50, lim // 50, size=3872)   # noise floor
-    iq = iq.astype(np.int16)
-    mag_r, ml_r, mp_r = Reference().convert_sc16(iq, q11)
+    return iq.astype(np.int16)
+
+
+@pytest.mark.parametrize("q11", [False, True])
+def test_oracle_sc16_converters_match_reference(q11):
+    """SURVEY 8(f) row 3: convert_sc16_nodc (convert.c:212-250) / convert_sc16q11_nodc (:329-367), magnitudes and the two
+    sequential float accumulators, against the reference's own converters reached through init_converter."""
+    want = reference_runs()[f"sc16/{int(q11)}"]
+    iq = sc16_input(q11); n = iq.size // 2
     mag_o, sl_o, sp_o = Oracle.convert_sc16(iq, q11)
-    assert np.array_equal(mag_r, mag_o) and mag_o.max() == 65535 and mag_o[32:64].min() == 0
-    assert float(np.float32(sl_o) / np.float32(n)) == ml_r and float(np.float32(sp_o) / np.float32(n)) == mp_r
+    assert digest(mag_o) == want["mag"] and mag_o.max() == 65535 and mag_o[32:64].min() == 0
+    assert float(np.float32(sl_o) / np.float32(n)) == want["mean_level"] and float(np.float32(sp_o) / np.float32(n)) == want["mean_power"]
 
 
 def _to_sc16(iq8: np.ndarray, q11: bool, seed: int) -> np.ndarray:
@@ -298,54 +318,59 @@ def _to_sc16(iq8: np.ndarray, q11: bool, seed: int) -> np.ndarray:
     return np.clip(v, -2048 if q11 else -32768, 2047 if q11 else 32767).astype(np.int16)
 
 
-@needs_ref
-@pytest.mark.parametrize("q11,buf", [(False, 65536), (True, 20000)])
+def modeac_sc16_input(q11):
+    return _to_sc16(synth.modeac_stream(31 + q11, 1_200_000), q11, 9)
+
+
+@pytest.mark.parametrize("q11,buf", MODEAC_SC16_CASES)
 def test_oracle_modeac_with_converter_levels_matches_reference(q11, buf):
     """demodulate2400AC takes its noise floor from mag_buf.mean_level / mean_power (demod_2400.c:580-581); for an sc16 frontend
     those are float-accumulated means (convert.c:243-249), not the exact integer sums: the reference's converter + the
     reference's demodulate2400AC against the oracle's converter + oracle_demodulate2400AC_levels."""
-    iq16 = _to_sc16(synth.modeac_stream(31 + q11, 1_200_000), q11, 9)
-    ar = Reference().run_stream_ac_sc16(iq16, buf, q11)
+    want = reference_runs()[f"modeac_sc16/{int(q11)}/{buf}"]
     o = Oracle()
-    ao = o.run_stream_ac_sc16(iq16, buf, q11)
-    assert len(ar) > 80 and len(ar) == len(ao)
-    for f in ("timestamp", "modeac", "buffer_idx"):      # the reference harness cannot see f1_sample
-        assert np.array_equal(ar[f], ao[f]), f
-    assert o.stats()["demod_modeac"] == len(ar)
+    ao = o.run_stream_ac_sc16(modeac_sc16_input(q11), buf, q11)
+    assert want["n"] > 80 and len(ao) == want["n"] == o.stats()["demod_modeac"]
+    # the reference harness cannot see f1_sample
+    problems = diff_digests(record_digests(ao, ("timestamp", "modeac", "buffer_idx")), want["replies"])
+    assert not problems, "\n".join(problems)
 
 
-@needs_ref
+def dropped_input():
+    return synth.mixed_stream(21, 6 * 65536)
+
+
 def test_dropped_samples_raise_the_threshold_to_75():
     """demod_2400.c:334-338: while stats_15min.samples_dropped is set the reference uses max(75, preambleThreshold); the
     boundary exposes that as a threshold the caller sets between buffers."""
-    iq = synth.mixed_stream(21, 6 * 65536)
-    ref = Reference(preamble_threshold=58)
-    ref.set_samples_dropped(3)
-    fr = ref.run_stream(iq, 65536)[0]
+    want = reference_runs()["dropped_samples"]
+    iq = dropped_input()
     o = Oracle(preamble_threshold=58)
     o.set_preamble_threshold(75)
     fo, _ = o.run_stream(iq, 65536)
     o58 = Oracle(preamble_threshold=58)
     o58.run_stream(iq, 65536)
-    assert len(fr) > 50 and not diff_frames(fo, fr, fields=("timestamp", "msg", "score"))
-    assert ref.stats()[0]["demod_preambles"] == o.stats()["demod_preambles"] < o58.stats()["demod_preambles"]
+    assert want["n_frames"] > 50 and not diff_digests(record_digests(fo, ("timestamp", "msg", "score")), want["frames"])
+    assert want["demod_preambles"] == o.stats()["demod_preambles"] < o58.stats()["demod_preambles"]
 
 
-@needs_ref
+def syndrome_ffffff_input():
+    z = np.load(Path(__file__).resolve().parent / "golden" / "regress" / "syndrome_ffffff.npz")
+    return z["iq"], int(z["preamble_threshold"])
+
+
 def test_reference_rejects_the_all_ones_syndrome():
     """tests/golden/regress/syndrome_ffffff.npz holds a DF17 candidate with syndrome 0xFFFFFF (no single-bit error has it): the
     reference and the oracle both find nothing to accept in that window (the CUDA path once did, see tests/test_gpu_edges.py)."""
-    z = np.load(Path(__file__).resolve().parent / "golden" / "regress" / "syndrome_ffffff.npz")
-    iq, thr = z["iq"], int(z["preamble_threshold"])
-    ref, o = Reference(preamble_threshold=thr), Oracle(preamble_threshold=thr)
-    fr = ref.run_stream(iq, 65536)[0]
+    want = reference_runs()["syndrome_ffffff"]
+    iq, thr = syndrome_ffffff_input()
+    o = Oracle(preamble_threshold=thr)
     fo, _ = o.run_stream(iq, 65536)
-    assert len(fr) == len(fo) == 0
-    assert ref.stats()[0]["demod_preambles"] == o.stats()["demod_preambles"] > 10
+    assert want["n_frames"] == len(fo) == 0
+    assert want["demod_preambles"] == o.stats()["demod_preambles"] > 10
     assert Oracle.diagnose1(0xFFFFFF, 112) < 0 and Oracle.diagnose1(0xFFFFFF, 56) < 0
 
 
-@needs_ref
 def test_aggressive_error_tables_match_reference():
     """--aggressive (nfix_crc = 2, crc.c:180-378 with max_correct 2 / max_detect 4): the oracle's table — preparation, the
     demodulator path does not use it yet — holds exactly the syndromes the reference's modesChecksumDiagnose knows, with the same
@@ -355,14 +380,10 @@ def test_aggressive_error_tables_match_reference():
     L = Oracle.lib()
     L.oracle_crc_table2_digest.argtypes = [C.c_int, C.POINTER(C.c_uint64)]
     L.oracle_crc_diagnose2.argtypes = [C.c_uint32, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
-    ref = Reference()
-    ref.L.ref_crc_table2_digest.argtypes = [C.c_int, C.POINTER(C.c_uint64)]
     for bits, n_expected in ((56, 51 + 1275), (112, 107 + 3724)):
-        do, dr = C.c_uint64(), C.c_uint64()
+        do = C.c_uint64()
         no = L.oracle_crc_table2_digest(bits, C.byref(do))
-        nr = ref.L.ref_crc_table2_digest(bits, C.byref(dr))
-        assert no == nr == n_expected and do.value == dr.value
-    Reference()        # the digest call re-initialised the reference's tables for two-bit correction: put them back
+        assert [no, do.value] == reference_runs()["crc_table2_digest"][str(bits)] and no == n_expected
     b0, b1 = C.c_int(), C.c_int()
     assert L.oracle_crc_diagnose2(0x3935EA, 112, C.byref(b0), C.byref(b1)) == -2          # bit 0 is a DF bit: never corrected
     assert L.oracle_crc_diagnose2(0xFFF409, 112, C.byref(b0), C.byref(b1)) == 1 and (b0.value, b1.value) == (87, -1)
